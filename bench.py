@@ -2,6 +2,7 @@
 """bench.py -- ALS user+item row-updates/sec at f=64 (BASELINE.json metric) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2] [--scale S]
+                    [--dump-outputs DIR]
 
 A "step" is one ALS iteration of the hot path (user half + item half, each = Gramian + fused
 per-row Cholesky solve [+ factor all-gather at N > 1]) over the synthetic last.fm-shaped matrix C2
@@ -14,6 +15,7 @@ One process per GPU (torchrun-compatible env: RANK / LOCAL_RANK / WORLD_SIZE / M
 rank 0 prints exactly one JSON line.  --impl reference times the reference's own Cython/OpenMP CPU
 path (oracle/_ref when it was built where /root/reference exists, else the C restatement) on a
 bounded row sample of the same workload, on rank 0 only.
+--dump-outputs DIR writes what the timed path computed in its last step as DIR/<name>.npy (see dump_outputs).
 """
 import argparse
 import json
@@ -32,6 +34,7 @@ import numpy as np  # noqa: E402
 METRIC = "ALS user+item row-updates/sec at f=64"
 UNIT = "row-updates/s"
 E2E_ITERS = 3
+DUMP_BYTES = 60_000_000  # what --dump-outputs may write in all: under 64 MB with the .npy headers
 
 
 def metric_name(cfg):
@@ -50,7 +53,13 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--trace-e2e", action="store_true", help="cProfile of the last end-to-end fit, to stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
+    return args
 
 
 # --------------------------------------------------------------------------------------- helpers
@@ -171,6 +180,18 @@ class ClockSampler:
             pass
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "samples_nvidia_smi": n_smi, "reasons": sorted(reasons)}
+
+
+def dump_outputs(path, arrays):
+    """Writes each 2-D float32 / float64 array as <path>/<name>.npy.  An array above its share of DUMP_BYTES keeps a
+    sample of its rows drawn with a fixed seed, in row order: runs with the same arguments write the same rows."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def pinned_csr(Cui):
@@ -368,6 +389,8 @@ def run_ours(args):
     prof = ctx.profile_read()
     ctx.profile(False)
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs and rank == 0:  # every rank holds both factor matrices whole
+        dump_outputs(args.dump_outputs, {"user_factors": X.download(), "item_factors": Y.download()})
     ms_max = pg.allreduce_max(ms) if world > 1 else ms
     value = (users + items) * args.steps / (ms_max * 1e-3)
 
@@ -623,13 +646,15 @@ def run_topk(args):
     t0 = time.perf_counter()
     for step in range(warm, warm + args.steps):
         lo, rows = batch_rows(step)
-        _lib.topk(ctx, di, dq, k, query_rows=rows, liked=liked_dev[lo])
+        ids, scores = _lib.topk(ctx, di, dq, k, query_rows=rows, liked=liked_dev[lo])
     ctx.sync()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     prof = ctx.profile_read()
     ctx.profile(False)
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"ids": ids.astype(np.float64), "scores": scores})
     k_ms, k_n = prof["topk"]
     ms = k_ms  # device time of the fused kernel(s): CUDA events around each launch on the library's stream
     value = batch * args.steps / (ms * 1e-3)

@@ -5,6 +5,9 @@ oracle/build_ref.py from /root/reference).  Run where /root/reference exists:
 
 Inputs are NOT stored: every case is rebuilt from implicit_b200.synthetic with the seed recorded in
 the file, so a fixture is (recipe, expected outputs of the reference).  Outputs are float32.
+
+port_vs_ref.npz (written alone with --port-vs-ref) holds the reference's side of tests/test_oracle.py's port-vs-
+reference checks; their warm states are reference outputs too, so they are stored, for a sample of the rows.
 """
 import os
 import sys
@@ -12,10 +15,12 @@ import sys
 os.environ.setdefault("OPENBLAS_NUM_THREADS", "1")
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import numpy as np  # noqa: E402
 
 import oracle  # noqa: E402
+from helpers import REF_ROWS, TIES_K, WIDE_ROWS, ref_half_case, ref_wide_case, ties_case  # noqa: E402
 from implicit_b200 import synthetic  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -54,7 +59,37 @@ def main():
         np.savez_compressed(os.path.join(HERE, name + ".npz"), X=X, Y=Y, Xh=Xh, loss=np.float64(loss), topk_ids=ids,
                             topk_scores=scores, **{"recipe_" + k: np.asarray(v) for k, v in rc.items()})
         print(name, "loss", loss, X.shape, Y.shape)
+    port_vs_ref()
+
+
+def port_vs_ref():
+    """tests/golden/port_vs_ref.npz: what tests/test_oracle.py compares the C restatement with."""
+    ref = oracle.get("ref")
+    out = {}
+    n = REF_ROWS
+    for name, use_cg in (("chol", False), ("cg", True)):
+        # one half from the reference's own warm state (two iterations)
+        Cui, X, Y = ref_half_case()
+        oracle.fit(Cui, X, Y, iterations=2, use_cg=use_cg, kind="ref")
+        Xh = X.copy()
+        if use_cg:
+            ref.least_squares_cg(Cui, Xh, Y, 0.01, cg_steps=3)
+        else:
+            ref.least_squares(Cui, Xh, Y, 0.01)
+        out.update({f"{name}_Y": Y, f"{name}_X": X[:n], f"{name}_Xh": Xh[:n],
+                    f"{name}_loss": np.float64(ref.calculate_loss(Cui[:n], Xh[:n], Y, 0.01))})
+    Cui, X, Y = ref_wide_case()
+    n = WIDE_ROWS
+    ref.least_squares_cg(Cui, X, Y, 0.01, cg_steps=3)
+    ids, scores = ref.topk(Y, X[:20], 7, filter_query_items=Cui[:20])
+    out.update(wide_Xh=X[:n], wide_loss=np.float64(ref.calculate_loss(Cui[:n], X[:n], Y, 0.01)), wide_topk_ids=ids,
+               wide_topk_scores=scores)
+    items, q = ties_case()
+    for k in TIES_K:
+        out[f"ties_ids_k{k}"], out[f"ties_scores_k{k}"] = ref.topk(items, q, k)
+    np.savez_compressed(os.path.join(HERE, "port_vs_ref.npz"), **out)
+    print("port_vs_ref", sorted(out))
 
 
 if __name__ == "__main__":
-    main()
+    port_vs_ref() if "--port-vs-ref" in sys.argv else main()

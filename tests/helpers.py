@@ -46,6 +46,38 @@ def load_golden(name):
     return rc, Cui, X0, Y0, z
 
 
+# ----------------------------------------------------------------------------- port-vs-reference fixtures
+#: tests/golden/port_vs_ref.npz keeps the factor rows of the first REF_ROWS / WIDE_ROWS users only: rows solve
+#: independently, and power_law_csr permutes the users, so the first rows are a random sample of the matrix.
+REF_ROWS = 100
+WIDE_ROWS = 48
+TIES_K = (1, 5, 32, 250)
+
+
+def ref_half_case():
+    """500 x 300, 6000 nnz with 5 % negative weights, 48 factors, from the initial factors."""
+    Cui = synthetic.power_law_csr(500, 300, 6000, 77, negative_fraction=0.05)
+    X0, Y0 = synthetic.initial_factors(500, 300, 48)
+    return Cui, X0, Y0
+
+
+def ref_wide_case():
+    """192 factors (the widths of tests/test_gpu_wide.py) from random factors."""
+    Cui = synthetic.power_law_csr(200, 150, 3000, 78, negative_fraction=0.05)
+    rng = np.random.default_rng(5)
+    X = (rng.standard_normal((200, 192)) * 0.1).astype(np.float32)
+    Y = (rng.standard_normal((150, 192)) * 0.1).astype(np.float32)
+    return Cui, X, Y
+
+
+def ties_case():
+    """Small-integer items and queries: many exact score ties."""
+    rng = np.random.default_rng(5)
+    items = rng.integers(0, 4, size=(200, 3)).astype(np.float32)
+    q = rng.integers(0, 3, size=(17, 3)).astype(np.float32)
+    return items, q
+
+
 # ----------------------------------------------------------------------------- evaluation fixtures
 class TableModel:
     """Stands in for a fitted model: `recommend` returns precomputed ranked ids (no GPU involved)."""
@@ -71,3 +103,17 @@ def eval_case(users, items, K, seed):
     test = sp.csr_matrix((np.ones(len(indices), dtype=np.float32), indices, indptr), shape=(users, items))
     train = sp.random(users, items, density=0.05, format="csr", dtype=np.float32, random_state=seed)
     return TableModel(table), train, test
+
+
+def eval_second_cutoff(K):
+    """The cutoff tests/golden/eval_ref.npz holds the reference's metrics at, besides each case's own K."""
+    return max(1, K // 2)
+
+
+LEAVE_K_OUT_K = (1, 3)
+
+
+def leave_k_out_ratings():
+    import scipy.sparse as sp
+
+    return sp.random(100, 100, density=0.5, format="csr", dtype=np.float32, random_state=5).tocoo()

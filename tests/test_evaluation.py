@@ -1,18 +1,18 @@
 """Ranking evaluation (SURVEY.md 8(f) N4; implicit/evaluation.pyx:366-475).
 
 CPU part: the metric arithmetic of implicit_b200.evaluation and of the oracle restatement against the
-golden values produced by the reference's own compiled module, with a table of precomputed ids standing in
-for the model.  GPU part: the real model driving the fused top-k kernel through `recommend`."""
+golden values produced by the reference's own compiled module (eval_metrics.npz, eval_ref.npz), with a table of
+precomputed ids standing in for the model.  GPU part: the real model driving the fused top-k kernel through `recommend`."""
 import os
 
 import numpy as np
 import pytest
 
-import oracle
-from helpers import eval_case
+from helpers import LEAVE_K_OUT_K, eval_case, eval_second_cutoff, leave_k_out_ratings
 from oracle import evaluation_oracle
 
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "eval_metrics.npz"))
+REF = np.load(os.path.join(os.path.dirname(__file__), "golden", "eval_ref.npz"))
 CASES = sorted({k.split("_")[0] for k in GOLD.files})
 KEYS = ("precision", "map", "ndcg", "auc")
 
@@ -32,14 +32,12 @@ def test_oracle_restatement_matches_golden(name):
 
 @pytest.mark.parametrize("name", CASES)
 def test_oracle_restatement_matches_compiled_reference(name):
-    if not oracle.have_ref_evaluation():
-        pytest.skip("oracle/_ref/evaluation not built")
+    """The same cases at a second cutoff, below the length of the ranked lists."""
     rc = _recipe(name)
     model, train, test = eval_case(**rc)
-    exp = oracle.ref_evaluation().ranking_metrics_at_k(model, train, test, K=rc["K"], show_progress=False)
-    got = evaluation_oracle.ranking_metrics_at_k(model, train, test, K=rc["K"])
+    got = evaluation_oracle.ranking_metrics_at_k(model, train, test, K=eval_second_cutoff(rc["K"]))
     for k in KEYS:
-        assert got[k] == pytest.approx(exp[k], rel=1e-12)
+        assert got[k] == pytest.approx(float(REF[f"{name}_{k}"]), rel=1e-12)
 
 
 @pytest.mark.parametrize("name", CASES)
@@ -74,17 +72,11 @@ def test_train_test_split_matches_golden(name):
 
 
 # ---- leave_k_out_split: the reference's own property tests (tests/evaluation_test.py:30-100)
-def _ratings():
-    import scipy.sparse as sp
-
-    return sp.random(100, 100, density=0.5, format="csr", dtype=np.float32, random_state=5).tocoo()
-
-
-@pytest.mark.parametrize("K", [1, 3])
+@pytest.mark.parametrize("K", LEAVE_K_OUT_K)
 def test_leave_k_out_split_contract(K):
     from implicit_b200 import evaluation
 
-    mat = _ratings()
+    mat = leave_k_out_ratings()
     train, test = evaluation.leave_k_out_split(mat, K=K, random_state=1)
     assert train.shape == mat.shape and test.shape == mat.shape          # :30-38
     assert ((train + test) - mat).nnz == 0                                # :41-49
@@ -94,15 +86,13 @@ def test_leave_k_out_split_contract(K):
     assert np.all(held[counts > K + 1] == K) and np.all(held[counts <= K + 1] == 0)
     t2, _ = evaluation.leave_k_out_split(mat, K=K, random_state=1)       # seeded
     assert (t2 != train).nnz == 0
-    if oracle.have_ref_evaluation():  # same contract from the reference's compiled module
-        rt, rs = oracle.ref_evaluation().leave_k_out_split(mat, K=K)
-        assert ((rt + rs) - mat).nnz == 0 and np.array_equal(np.diff(rs.indptr), held)
+    np.testing.assert_array_equal(REF[f"leave_k_out_held_K{K}"], held)  # what the reference's compiled module holds out
 
 
 def test_leave_k_out_split_train_only_and_errors():
     from implicit_b200 import evaluation
 
-    mat = _ratings()
+    mat = leave_k_out_ratings()
     train, test = evaluation.leave_k_out_split(mat, K=1, train_only_size=0.8, random_state=2)
     train_only = ~np.isin(np.unique(train.tocoo().row), test.tocoo().row)
     assert train_only.sum() == int(train.shape[0] * 0.8)                  # :69-76

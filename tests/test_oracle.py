@@ -1,15 +1,19 @@
 """CPU-only: pins the oracle (oracle/als_oracle.c) against
   (1) the golden vectors generated from the reference's own compiled Cython (tests/golden/),
-  (2) that compiled reference itself when oracle/_ref is present in this checkout,
+  (2) that compiled reference's answers on the same inputs (tests/golden/port_vs_ref.npz),
   (3) the known-answer / property tests the reference holds for this path."""
+import os
+
 import numpy as np
 import pytest
 from scipy.sparse import csr_matrix
 
 import oracle
-from helpers import CHOL_MAX, golden_cases, load_golden, row_err
+from helpers import (CHOL_MAX, GOLDEN, REF_ROWS, TIES_K, WIDE_ROWS, golden_cases, load_golden, ref_half_case,
+                     ref_wide_case, row_err, ties_case)
 
 PORT = oracle.get("port")
+REF = np.load(os.path.join(GOLDEN, "port_vs_ref.npz"))
 
 
 @pytest.mark.parametrize("name", golden_cases())
@@ -53,47 +57,32 @@ def test_port_loss_and_topk_match_golden(name):
         assert np.abs(scores[diff] - z["topk_scores"][diff]).max() < 1e-6
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built in this checkout")
 @pytest.mark.parametrize("use_cg", [False, True])
 def test_port_matches_compiled_reference(use_cg):
-    from implicit_b200 import synthetic
-
-    ref = oracle.get("ref")
-    Cui = synthetic.power_law_csr(500, 300, 6000, 77, negative_fraction=0.05)
-    X0, Y0 = synthetic.initial_factors(500, 300, 48)
-    # warm state from the reference, then one half with each implementation
-    Xw, Yw = X0.copy(), Y0.copy()
-    oracle.fit(Cui, Xw, Yw, iterations=2, use_cg=use_cg, kind="ref")
-    Xa, Xb = Xw.copy(), Xw.copy()
+    """One half from the reference's warm state (two reference iterations), against the reference's half."""
+    name = "cg" if use_cg else "chol"
+    Cui = ref_half_case()[0][:REF_ROWS]
+    Yw, Xa = REF[f"{name}_Y"], REF[f"{name}_Xh"]
+    Xb = REF[f"{name}_X"].copy()
     if use_cg:
-        ref.least_squares_cg(Cui, Xa, Yw, 0.01, cg_steps=3)
         PORT.least_squares_cg(Cui, Xb, Yw, 0.01, cg_steps=3)
     else:
-        ref.least_squares(Cui, Xa, Yw, 0.01)
         PORT.least_squares(Cui, Xb, Yw, 0.01)
     assert row_err(Xb, Xa).max() < 1e-5
-    assert PORT.calculate_loss(Cui, Xa, Yw, 0.01) == pytest.approx(ref.calculate_loss(Cui, Xa, Yw, 0.01), rel=1e-6)
+    assert PORT.calculate_loss(Cui, Xa, Yw, 0.01) == pytest.approx(float(REF[f"{name}_loss"]), rel=1e-6)
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built in this checkout")
 def test_port_matches_compiled_reference_on_a_wide_model():
     """192 factors (the widths of tests/test_gpu_wide.py): the checker itself must not care about the width."""
-    from implicit_b200 import synthetic
-
-    ref = oracle.get("ref")
-    Cui = synthetic.power_law_csr(200, 150, 3000, 78, negative_fraction=0.05)
-    rng = np.random.default_rng(5)
-    X = (rng.standard_normal((200, 192)) * 0.1).astype(np.float32)
-    Y = (rng.standard_normal((150, 192)) * 0.1).astype(np.float32)
-    Xa, Xb = X.copy(), X.copy()
-    ref.least_squares_cg(Cui, Xa, Y, 0.01, cg_steps=3)
+    Cui, X, Y = ref_wide_case()
+    Cui, Xa = Cui[:WIDE_ROWS], REF["wide_Xh"]
+    Xb = X[:WIDE_ROWS].copy()
     PORT.least_squares_cg(Cui, Xb, Y, 0.01, cg_steps=3)
     assert row_err(Xb, Xa).max() < 1e-5
-    assert PORT.calculate_loss(Cui, Xa, Y, 0.01) == pytest.approx(ref.calculate_loss(Cui, Xa, Y, 0.01), rel=1e-6)
-    ia, sa = ref.topk(Y, Xa[:20], 7, filter_query_items=Cui[:20])
+    assert PORT.calculate_loss(Cui, Xa, Y, 0.01) == pytest.approx(float(REF["wide_loss"]), rel=1e-6)
     ib, sb = PORT.topk(Y, Xa[:20], 7, filter_query_items=Cui[:20])
-    np.testing.assert_allclose(sb, sa, rtol=1e-5, atol=1e-7)
-    assert (ia == ib).mean() > 0.98
+    np.testing.assert_allclose(sb, REF["wide_topk_scores"], rtol=1e-5, atol=1e-7)
+    assert (REF["wide_topk_ids"] == ib).mean() > 0.98
 
 
 # ---- the reference's own known-answer tests for this path ------------------------------------------
@@ -161,14 +150,9 @@ def test_select_tie_semantics():
     assert ids.tolist() == [[1, 0, 0, 0]] and sc.tolist() == [[1.0, 1.0, 0.0, 0.0]]
 
 
-@pytest.mark.skipif(not oracle.have_ref(), reason="oracle/_ref not built in this checkout")
 def test_select_matches_compiled_reference_on_ties():
-    ref = oracle.get("ref")
-    rng = np.random.default_rng(5)
-    items = rng.integers(0, 4, size=(200, 3)).astype(np.float32)  # many exact ties
-    q = rng.integers(0, 3, size=(17, 3)).astype(np.float32)
-    for k in (1, 5, 32, 250):
-        a = ref.topk(items, q, k)
+    items, q = ties_case()
+    for k in TIES_K:
         b = PORT.topk(items, q, k)
-        np.testing.assert_array_equal(a[0], b[0])
-        np.testing.assert_array_equal(a[1], b[1])
+        np.testing.assert_array_equal(REF[f"ties_ids_k{k}"], b[0])
+        np.testing.assert_array_equal(REF[f"ties_scores_k{k}"], b[1])
