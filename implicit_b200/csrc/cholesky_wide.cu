@@ -172,7 +172,13 @@ cholesky_wide_kernel(const int32_t *__restrict__ indices, const float *__restric
   }
 }
 
-__global__ void init_bad_row(long long *bad_row) { bad_row[0] = LLONG_MAX; }
+// Like init_solver_scalars (cholesky.cu): [1] keeps the first bad row of every half since the last als_solver_status.
+// Resetting [0] alone lost a failed half of 65..128 factors that the asynchronous (multi-GPU) fit had not collected
+// yet: the next half erased it and als_solver_status reported nothing (tests/test_gpu_width_sweep.py, f = 80, 128).
+__global__ void init_bad_row(long long *bad_row) {
+  if (bad_row[0] < bad_row[1]) bad_row[1] = bad_row[0];
+  bad_row[0] = LLONG_MAX;
+}
 
 template <int T>
 int run_wide(als_ctx *ctx, const als_csr *Cm, als_factors *X, const als_factors *Y) {
